@@ -135,6 +135,14 @@ def cpu_sample(om, np, n_decode: int, prompt=None, forced=None, tp: int = 1):
     return t_prefill, t_decode, toks, logits
 
 
+def dump_outputs(out_dir, arrays, np):
+    """--dump-outputs: write what the timed path returned in its last step as <name>.npy (float64 holds every
+    token id exactly), so that two builds run with the same arguments can be compared output for output"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
 def bf16_ulps(a, b, np):
     """distance in bf16 ulps between two arrays of bf16-valued float32 (monotone integer map of the bit patterns)"""
     def key(x):
@@ -195,7 +203,7 @@ def run_reference(a):
     t0 = time.perf_counter()
     done = 0
     for _ in range(a.steps):
-        tp, td, _, _ = cpu_sample(om, np, n_dec)
+        tp, td, toks, _ = cpu_sample(om, np, n_dec)
         t_dec_total += td
         t_pre_total += tp
         done += 1
@@ -220,6 +228,8 @@ def run_reference(a):
                          "prefill_s": round(t_pre_total / a.steps, 3)},
         "e2e": {"value": round(val, 4), "unit": "tokens/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"tokens": toks}, np)
     print(json.dumps(line), flush=True)
 
 
@@ -366,7 +376,7 @@ def run_decode(a):
         launches = ctx.launch_count() - launches0
         assert gen_k == gen, "generation is not reproducible run to run"
         dec_ms, wall = env.max_over_ranks(dec_ms, wall)
-        return dict(ctx=ctx, tokens=gen, dec_ms=dec_ms, wall=wall, pre_s=pre_s, graphed=graphed, clocks=clocks, launches=launches,
+        return dict(ctx=ctx, tokens=gen_k, dec_ms=dec_ms, wall=wall, pre_s=pre_s, graphed=graphed, clocks=clocks, launches=launches,
                     value=n_steps * N_DECODE / (dec_ms / 1e3), engine=ctx.uses_engine())
 
     try:
@@ -539,6 +549,9 @@ def run_decode(a):
             "e2e": e2e, "other_acc_mode": other, "other_collective": other_coll, "cpu_baseline": cpu, "parity": parity,
             "model_load_s": round(env.t_load, 2),
         }
+        if a.dump_outputs:
+            # the generation of the last timed step: token #1 from the prefill, then the 127 decoded tokens
+            dump_outputs(a.dump_outputs, {"tokens": gen_tokens}, np)
         print(json.dumps(line), flush=True)
     env.close()
 
@@ -598,6 +611,8 @@ def run_prefill(a):
                          "what": "whole call: linears + causal SDPA + last-row LM head, algorithmic flops / wall time (H2D/D2H included)"},
             "e2e": {"value": round(S / per, 1), "unit": "tokens/s", "h2d_bytes_per_step": S * 4, "d2h_bytes_per_step": 4},
             "cpu_baseline": None, "parity": parity, "next_token": int(nxt)}
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {"next_token": [nxt]}, np)
     print(json.dumps(line), flush=True)
     ctx.close()
     env.close()
@@ -677,6 +692,9 @@ def run_batch8(a):
                 "e2e": {"value": round(h["value"], 1), "unit": "tokens/s", "h2d_bytes_per_step": 64 * N_DECODE, "d2h_bytes_per_step": 32 * N_DECODE},
                 "other_acc_mode": {"acc": [k for k in res if k != a.acc][0], "value": round([v for k, v in res.items() if k != a.acc][0]["value"], 1)},
                 "cpu_baseline": None, "parity": parity}
+        if a.dump_outputs:
+            # [8 sequences, 128 tokens] of the headline arm's last timed generation
+            dump_outputs(a.dump_outputs, {"tokens": h["toks"]}, np)
         print(json.dumps(line), flush=True)
     env.close()
 
@@ -697,7 +715,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / parity legs")
     ap.add_argument("--parity-tokens", type=int, default=128, help="generated tokens compared with the oracle (teacher-forced)")
     ap.add_argument("--parity", action="store_true", help="prefill2048: also run the oracle's S=2048 prefill (minutes of CPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the token ids the timed path returned in its last step as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.impl == "reference":
         return run_reference(a)
     a.warmup = max(a.warmup, 3)

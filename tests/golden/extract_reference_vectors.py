@@ -6,6 +6,7 @@ however hold literal known answers for this path (SURVEY 8c).  This script parse
 under /root/reference (read-only) and records file:line for each, so the committed fixture is provably the
 reference's data and not a transcription.  Run here:  python tests/golden/extract_reference_vectors.py
 (/root/reference does not exist on the GPU box; tests only read the committed JSON.)"""
+import hashlib
 import json
 import os
 import re
@@ -13,7 +14,15 @@ import sys
 
 REF = os.environ.get("LNB_REFERENCE_DIR", "/root/reference")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "reference_vectors.json")
+# digest of what was extracted, kept beside the fixture: without a reference checkout the tests can still tell that the
+# fixture is the extraction and was not edited by hand
+DIGEST = os.path.join(os.path.dirname(OUT), "reference_vectors.sha256")
 NUM = r"[-+]?(?:\d+\.\d*|\.\d+|\d+)(?:[eE][-+]?\d+)?"
+
+
+def digest(vectors) -> str:
+    """SHA-256 of the extracted vectors in canonical JSON (sorted keys, no whitespace)"""
+    return hashlib.sha256(json.dumps(vectors, sort_keys=True, separators=(",", ":")).encode()).hexdigest()
 
 
 def read(rel):
@@ -179,7 +188,9 @@ def main():
     with open(OUT, "w") as f:
         json.dump(out, f, indent=1, sort_keys=True)
         f.write("\n")
-    print("wrote", OUT)
+    with open(DIGEST, "w") as f:
+        f.write(digest(out) + "\n")
+    print("wrote", OUT, "and", DIGEST)
 
 
 if __name__ == "__main__":
